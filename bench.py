@@ -6,6 +6,7 @@ steps per env).  The metric is BASELINE.json's: env steps/sec, one env step = on
 (src/experiment/serial.cpp:53-70).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload C1..C4] [--no-extras]
+                    [--dump-outputs DIR]
 
 N > 1 is launched by torchrun (one rank per GPU); envs are sharded by rank, independent policies need no data-path
 collective ("scaling": "weak").  The headline is C1 (BASELINE.json configs[1]) per GPU; the line also carries, under
@@ -42,6 +43,11 @@ WORKLOADS = {
 # 32-byte sectors = 26 % of the copy bandwidth): the DRAM ceiling of a tile-coded evaluation whose table does not fit
 # on chip.  A coalesced 32 KB window per step streams at 6.6-7.0 TB/s instead.
 DRAM_RANDOM_SECTORS_PER_S = 53.6e9
+# --dump-outputs: per-env arrays and the weight-table sample each stay under these sizes, so that the whole dump, index
+# arrays included, stays under 64 MB
+DUMP_ENV_BYTES = 24 << 20
+DUMP_THETA_BYTES = 16 << 20
+DUMP_SEED = 2024
 
 
 def engine_is_rounds(B, algo, shared, ticks_per_call):
@@ -128,6 +134,42 @@ def make_cfg(workload, n_envs, env_index0, source, args):
     cfg = config.from_dict(y, n_envs=n_envs, env_index0=env_index0, source=source, flow_seed=2024, dt_ms=1,
                            shared_policy=bool(w.get("shared")))
     return y, cfg
+
+
+def _sample(rng, n, cap):
+    """range(n) whole, or a fixed seeded sample of `cap` of its values in ascending order."""
+    import numpy as np
+    return np.arange(n) if n <= cap else np.sort(rng.choice(n, max(cap, 1), replace=False))
+
+
+def dump_outputs(m, cfg, algo, out_dir):
+    """Writes what a caller of the timed path can read back after its last step as out_dir/<name>.npy: every env's state
+    vector, reward, action and EnvStats fields, and the weight tables of a fixed, seeded sample of policies (all of them
+    are GBs at C1).  The same arguments give the same inputs, so two builds can be compared array by array."""
+    import numpy as np
+    from rl_markets_b200 import abi
+    os.makedirs(out_dir, exist_ok=True)
+    B, M, nv = cfg.n_envs, cfg.memory_size, cfg.n_state_vars
+    rng = np.random.default_rng(DUMP_SEED)
+    stat_names = [f for f, _ in abi.EnvStats._fields_]
+    envs = _sample(rng, B, DUMP_ENV_BYTES // (4 * nv + 8 * (3 + len(stat_names))))
+    out = {"env_index": envs.astype(np.float64),
+           "state": np.ctypeslib.as_array(m.state()).reshape(B, nv)[envs].astype(np.float32),
+           "reward": np.ctypeslib.as_array(m.rewards())[envs].astype(np.float64),
+           "action": np.ctypeslib.as_array(m.actions())[envs].astype(np.float64)}
+    st = np.ctypeslib.as_array(m.stats())[envs]
+    for f in stat_names:
+        out["stats_" + f] = st[f].astype(np.float64)
+    tables = 2 if algo in ("double_q_learn", "double_r_learn") else 1
+    policies = _sample(rng, 1 if cfg.shared_policy else B, DUMP_THETA_BYTES // (8 * tables * M))
+    cols = _sample(rng, M, DUMP_THETA_BYTES // (8 * tables * len(policies)))
+    theta = np.empty((len(policies), tables, len(cols)), dtype=np.float64)
+    for i, p in enumerate(policies):
+        for t in range(tables):
+            theta[i, t] = np.ctypeslib.as_array(m.theta(int(p), t))[cols]
+    out.update(theta=theta, theta_policy_index=policies.astype(np.float64), theta_column_index=cols.astype(np.float64))
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class Ctx:
@@ -237,6 +279,8 @@ def measure(ctx, name, args, steps, warmup, headline):
     if sampler:
         sampler.stop_flag = True
     m.sync()
+    if headline and args.dump_outputs and ctx.rank == 0:
+        dump_outputs(m, cfg, algo, args.dump_outputs)  # before the per-kernel pass below moves the state on
     c1 = m.counters()
     total_ms = evs[0].elapsed_time(evs[-1])
     steps_done, ticks_done, z_sum = c1.steps - c0.steps, c1.ticks - c0.ticks, c1.sum_traces - c0.sum_traces
@@ -603,6 +647,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-ticks", type=int, default=1200000)
     ap.add_argument("--ref-ticks", type=int, default=100000)
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the last one computed (rank 0's envs) as DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

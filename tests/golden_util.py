@@ -1,5 +1,6 @@
 """Loaders for tests/golden (fixtures generated from the compiled reference by tools/make_golden.py)."""
 import ctypes as C
+import hashlib
 import json
 import os
 import struct
@@ -48,6 +49,22 @@ def records(name):
     n = len(raw) // C.sizeof(abi.StepRecord)
     arr = (abi.StepRecord * n).from_buffer_copy(raw)
     return [arr[i] for i in range(n)], arr
+
+
+def record_digest(r):
+    """8-byte BLAKE2b of the fields abi.record_fields_equal compares, field by field (alignment bytes left out): equal
+    digests mean equal records.  Long reference runs are stored as digests_<name>.bin, one digest per record."""
+    h = hashlib.blake2b(digest_size=8)
+    for name, _t in abi.StepRecord._fields_:
+        if name != "pad":
+            f = getattr(abi.StepRecord, name)
+            h.update(C.string_at(C.addressof(r) + f.offset, f.size))
+    return h.digest()
+
+
+def digests(name):
+    raw = open(os.path.join(GOLD, "digests_%s.bin" % name), "rb").read()
+    return [raw[i:i + 8] for i in range(0, len(raw), 8)]
 
 
 def case_config(case, n_envs=1, env_index0=0, source=abi.SOURCE_GENERATOR):

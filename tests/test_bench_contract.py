@@ -61,6 +61,65 @@ def test_committed_scaling_and_reference_lines():
     assert ref["cpu_baseline"]["kind"] == "reference" and ref["cpu_baseline"]["cores"] >= 1
 
 
+class _FakeMarket:
+    """The read-back surface of lib.BatchedMarket that bench.dump_outputs uses, with values that name their origin."""
+
+    def __init__(self, cfg):
+        import numpy as np
+        self.cfg, self.np = cfg, np
+
+    def _arr(self, a):
+        return self.np.ctypeslib.as_ctypes(self.np.ascontiguousarray(a))
+
+    def state(self):
+        return self._arr(self.np.arange(self.cfg.n_envs * self.cfg.n_state_vars, dtype=self.np.float32))
+
+    def rewards(self):
+        return self._arr(self.np.arange(self.cfg.n_envs, dtype=self.np.float64) * 0.5)
+
+    def actions(self):
+        return self._arr(self.np.arange(self.cfg.n_envs, dtype=self.np.int32) % 9)
+
+    def stats(self):
+        from rl_markets_b200 import abi
+        st = (abi.EnvStats * self.cfg.n_envs)()
+        self.np.ctypeslib.as_array(st)["position"][:] = self.np.arange(self.cfg.n_envs)
+        return st
+
+    def theta(self, policy, table):
+        M = self.cfg.memory_size
+        return self._arr(self.np.arange(M, dtype=self.np.float64) + (2 * policy + table) * M)
+
+
+def test_dump_outputs_are_float_arrays_of_a_fixed_sample_under_64_mb(tmp_path):
+    """bench.py --dump-outputs: float32/float64 .npy files only, at most 64 MB in all, the same sample on every run."""
+    import types
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    shapes = [("double_q_learn", dict(n_envs=4096, memory_size=65536, n_state_vars=3, shared_policy=0)),      # C1, two tables
+              ("q_learn", dict(n_envs=300000, memory_size=1 << 22, n_state_vars=13, shared_policy=1))]     # larger than the budget
+    for algo, shape in shapes:
+        cfg = types.SimpleNamespace(**shape)
+        dirs = [tmp_path / ("%s_%d" % (algo, i)) for i in range(2)]
+        for d in dirs:
+            bench.dump_outputs(_FakeMarket(cfg), cfg, algo, str(d))
+        files = sorted(os.listdir(dirs[0]))
+        assert files == sorted(os.listdir(dirs[1])) and "theta.npy" in files and "reward.npy" in files
+        assert sum(os.path.getsize(dirs[0] / f) for f in files) <= 64 << 20
+        got = {f[:-4]: np.load(dirs[0] / f) for f in files}
+        for f in files:
+            assert got[f[:-4]].dtype in (np.float32, np.float64), f
+            assert np.array_equal(got[f[:-4]], np.load(dirs[1] / f)), f
+        envs = got["env_index"].astype(np.int64)
+        assert np.array_equal(got["stats_position"], envs) and np.array_equal(got["reward"], envs * 0.5)
+        pol, cols, th = got["theta_policy_index"].astype(np.int64), got["theta_column_index"].astype(np.int64), got["theta"]
+        tables = 2 if algo == "double_q_learn" else 1
+        assert th.shape == (len(pol), tables, len(cols)) and len(pol) >= 1
+        M = cfg.memory_size
+        assert np.array_equal(th[:, -1, :], cols[None, :] + (2 * pol[:, None] + tables - 1) * M)
+
+
 def test_reference_arm_runs_without_a_gpu():
     """`bench.py --impl reference` times the reference's CPU loop (oracle/_ref when built, else the oracle port)."""
     out = subprocess.check_output([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1",

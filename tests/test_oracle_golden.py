@@ -1,8 +1,7 @@
 """The CPU restatement (oracle/liblob_oracle.so) against the reference's own outputs.
 
 PINNING: tests/golden/* were produced by the UNMODIFIED reference compiled into oracle/_ref
-(tools/make_golden.py); when oracle/_ref exists (build container) the comparison is also
-run live on fresh seeds.  Everything is compared bitwise.
+(tools/make_golden.py).  Everything is compared bitwise.
 """
 import ctypes as C
 
@@ -178,7 +177,9 @@ def test_generators(oracle):
     assert [c for c in G.units()["rng"]["cases"] if c["seed"] == 1994][0]["rand"][:3] == [1261852369, 322867519, 980044188]
 
 
-_LIVE = [
+# whole reference runs of 4000 ticks of flow seed 123, env 0: other seeds than the manifest's, the R-learning agents,
+# Boltzmann, another venue's tick table and hours, random initial weights
+FLOW_SEED_123 = [
     ("double_q_learn", 8192, 31, {}),
     ("online_r_learn", 5003, 7, {"policy.eps_init": 0.2, "learning.beta": 0.02}),
     ("r_learn", 4096, 11, {"policy.type": "boltzmann", "policy.tau_init": 0.08, "policy.tau_floor": 0.01, "policy.tau_T": 10}),
@@ -186,22 +187,23 @@ _LIVE = [
 ]
 
 
-@pytest.mark.parametrize("algo,M,seed,over", _LIVE)
-def test_live_reference_when_built(oracle, algo, M, seed, over):
-    """In the build container the restatement is also checked against fresh runs of oracle/_ref (new seeds, the
-    R-learning agents, Boltzmann, another venue's tick table and hours, random initial weights)."""
-    if not oracle.have_ref():
-        pytest.skip("oracle/_ref not present on this machine; golden fixtures cover it")
+def flow_seed_123_case(algo, M, seed, over):
+    """(fixture name, reference yaml, config) of one FLOW_SEED_123 case."""
     y = config.example_dict(**{"learning.memory_size": M, "learning.algorithm": algo, "debug.random_seed": seed, **over})
-    cfg = config.from_dict(y, flow_seed=123)
+    return "flow123_%s_m%d" % (algo, M), y, config.from_dict(y, flow_seed=123)
+
+
+@pytest.mark.parametrize("algo,M,seed,over", FLOW_SEED_123)
+def test_whole_reference_runs_bitwise(oracle, algo, M, seed, over):
+    """The restatement against every record of a reference run (tests/golden/digests_flow123_*.bin, tools/make_golden.py)."""
+    name, _y, cfg = flow_seed_123_case(algo, M, seed, over)
     ticks = oracle.lib_generate(cfg, 0, 4000)
     port = oracle.run_port(cfg, 0, ticks)
-    ref = oracle.run_ref(y, 123, 0, 4000, want_theta=True, t0_ms=cfg.flow.t0_ms)
-    n = min(len(ref["records"]), port["steps"])
+    gold = G.digests(name)
+    n = min(len(gold), port["steps"])
     assert n > 800
-    for i in range(n):
-        bad = abi.record_fields_equal(ref["records"][i], port["records"][i])
-        assert not bad, "%s step %d: %r" % (algo, i, G.describe_diff(ref["records"][i], port["records"][i], bad))
+    bad = [i for i in range(n) if G.record_digest(port["records"][i]) != gold[i]]
+    assert not bad, "%s: steps %s differ from the reference's" % (algo, bad[:20])
 
 
 def test_book_scenarios(oracle):

@@ -7,12 +7,14 @@ which has no reference tree, can check against them).
   tests/golden/steps_<name>.bin    first N rlm_step_record of a reference run (oracle/_ref/ref_driver)
   tests/golden/bt_*_{profit_log,test_stats}.csv   the reference's own evaluation logs for the backtest cases
   tests/golden/manifest.json       the configs that produced them
+  (and, in tested_reference_runs, the fixtures single tests name themselves)
 """
 import ctypes as C
 import json
 import os
 import subprocess
 import sys
+from pathlib import Path
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -198,6 +200,49 @@ def main():
         print(c["name"], len(ref["records"]), "training records;", len(ref["test_records"]), "evaluation records")
     with open(os.path.join(GOLD, "manifest.json"), "w") as f:
         json.dump(manifest, f, indent=1)
+    tested_reference_runs()
+
+
+def tested_reference_runs():
+    """The reference outputs that single tests compare against, made with the tests' own cases and inputs:
+      digests_flow123_<algo>_m<M>.bin  tests/test_oracle_golden.py FLOW_SEED_123, every record of each run
+      digests_messy_flow77_*.bin       tests/test_ingest.py fresh_messy_pair, every record
+      file_pairing.json                tests/test_file_pairing.py REF_CALLS on each DIR_NAMES tree, root written {root}
+    Runs of a thousand records and more are kept as 8-byte digests per record (golden_util.record_digest)."""
+    import tempfile
+    import golden_util
+    import test_file_pairing as tfp
+    import test_ingest
+    import test_oracle_golden as tog
+
+    def write_digests(name, recs):
+        with open(os.path.join(GOLD, "digests_%s.bin" % name), "wb") as f:
+            for r in recs:
+                f.write(golden_util.record_digest(r))
+        print(name, len(recs), "records")
+    for case in tog.FLOW_SEED_123:
+        name, y, cfg = tog.flow_seed_123_case(*case)
+        write_digests(name, ol.run_ref(y, 123, 0, 4000, t0_ms=cfg.flow.t0_ms)["records"])
+    with tempfile.TemporaryDirectory() as d:
+        md, tas, y = test_ingest.fresh_messy_pair(d, ol.FLOW_CSV)
+        cfgp, dump = os.path.join(d, "cfg.yaml"), os.path.join(d, "steps.bin")
+        ol.write_ref_yaml(cfgp, y)
+        subprocess.check_output([ol.REF_DRIVER, "--config", cfgp, "--symbol", "AAL.L", "--md", md, "--tas", tas, "--dump", dump,
+                                 "--steps", "-1"])
+        raw = open(dump, "rb").read()
+    recs = (abi.StepRecord * (len(raw) // C.sizeof(abi.StepRecord))).from_buffer_copy(raw)
+    write_digests(test_ingest.FRESH_MESSY, recs)
+    pairing = {}
+    for md_name, tas_name in tfp.DIR_NAMES:
+        with tempfile.TemporaryDirectory() as d:
+            md, tas = tfp._tree(Path(d), md_name, tas_name)
+            calls = {}
+            for key, (verb, *rest) in tfp.REF_CALLS.items():
+                r = subprocess.run([os.path.join(ol.REF_DIR, "ref_files"), verb, md, tas] + rest, capture_output=True, text=True)
+                calls[key] = [r.returncode, [l.replace(d, "{root}").split("\t") for l in r.stdout.splitlines() if l]]
+        pairing["%s,%s" % (md_name, tas_name)] = calls
+    with open(os.path.join(GOLD, "file_pairing.json"), "w") as f:
+        json.dump(pairing, f, indent=1)
 
 
 if __name__ == "__main__":
