@@ -39,6 +39,7 @@ __host__ __device__ inline size_t ln_v_bytes(int is_double) { return (size_t)(is
 #ifndef UT_LOG2
 #define UT_LOG2 10  // 1024 slots, 512 entries per batch.  Measured: 256 or 512 slots cost more (longer probe chains in
 #endif               // every step's patch pass, extra batches on the launch's slowest warp) than the occupancy they buy
+static_assert(UT_LOG2 >= 7, "ut_clear writes UT_SLOTS / 128 int4 per lane: a smaller table would never be cleared");
 #define UT_SLOTS (1 << UT_LOG2)
 #define UT_MAX_ENTRIES (UT_SLOTS / 2)
 // learner scratch of one step: [V][tile table 2048][update table 8 * UT_SLOTS][q_pre 2*9 doubles][dec 6 doubles]

@@ -67,8 +67,16 @@ def digests(name):
     return [raw[i:i + 8] for i in range(0, len(raw), 8)]
 
 
+def learner_shapes():
+    """Whole reference runs at other action counts, gamma*lambda, trace caps and table sizes (digests_<name>.bin)."""
+    with open(os.path.join(GOLD, "learner_shapes.json")) as f:
+        return json.load(f)
+
+
 def case_config(case, n_envs=1, env_index0=0, source=abi.SOURCE_GENERATOR):
-    return config.from_dict(case["yaml"], n_envs=n_envs, env_index0=env_index0, flow_seed=case["flow_seed"], source=source)
+    c = config.from_dict(case["yaml"], n_envs=n_envs, env_index0=env_index0, flow_seed=case["flow_seed"], source=source)
+    c.trace_cap = case.get("trace_cap", 0)  # (the reference has no such key: it only sizes the device trace lists)
+    return c
 
 
 def hex_to_double(h):

@@ -8,6 +8,7 @@ which has no reference tree, can check against them).
   tests/golden/bt_*_{profit_log,test_stats}.csv   the reference's own evaluation logs for the backtest cases
   tests/golden/manifest.json       the configs that produced them
   (and, in tested_reference_runs, the fixtures single tests name themselves)
+  tests/golden/learner_shapes.json + digests_<name>.bin   LEARNER_SHAPE_CASES (`make_golden.py learner_shapes`: only these)
 """
 import ctypes as C
 import json
@@ -100,6 +101,50 @@ BACKTEST_CASES = [
     dict(name="bt_double_q_m8192", algo="double_q_learn", M=8192, flow_seed=23, env=5, ticks=1200, train_open_ticks=900,
          test=dict(flow_seed=24, env=5, ticks=1000, open_ticks=700), over={"learning.alpha_start": 0.01}),
 ]
+
+
+# The learner away from the example config: other action counts, gamma*lambda of 0 and 1 and long trace lists, an explicit
+# trace_cap, table sizes at the learner-selection boundaries (staged: single table, M*8 <= 64 KB, M even).  Every record of
+# each run is kept as digests_<name>.bin, the cases as learner_shapes.json -- not in manifest.json, whose consumers build
+# handles without a trace_cap.  min_traces / max_traces bound the longest trace list of the run, so that a case cannot
+# silently stop covering its path (several update-table drains per step, the rate == 0 skip).
+LEARNER_SHAPE_CASES = [
+    dict(name="a1_q_m8192", algo="q_learn", M=8192, flow_seed=5, env=0, ticks=3000, over={"learning.n_actions": 1},
+         min_traces=513),  # every action greedy: rate = gamma*lambda on every step; staged learner
+    dict(name="a2_sarsa_m2", algo="sarsa", M=2, flow_seed=5, env=1, ticks=2000, over={"learning.n_actions": 2}),
+    dict(name="a3_sarsa_m16384", algo="sarsa", M=16384, flow_seed=5, env=2, ticks=2000, over={"learning.n_actions": 3}),
+    dict(name="a5_q_m6002", algo="q_learn", M=6002, flow_seed=5, env=3, ticks=2000, over={"learning.n_actions": 5}),
+    dict(name="a7_dq_m4096", algo="double_q_learn", M=4096, flow_seed=5, env=4, ticks=2000, over={"learning.n_actions": 7}),
+    dict(name="a4_drl_m8209", algo="double_r_learn", M=8209, flow_seed=5, env=5, ticks=2000,
+         over={"learning.n_actions": 4, "policy.eps_init": 0.3, "learning.alpha_start": 0.01}),
+    dict(name="lam0_q", algo="q_learn", M=8192, flow_seed=5, env=6, ticks=2000, over={"learning.lambda": 0.0}, max_traces=32),
+    dict(name="lam0_sarsa", algo="sarsa", M=8192, flow_seed=5, env=7, ticks=2000, over={"learning.lambda": 0.0}, max_traces=32),
+    dict(name="longtr_sarsa_m65536", algo="sarsa", M=65536, flow_seed=5, env=8, ticks=3000,
+         over={"learning.gamma": 0.99, "learning.lambda": 0.97}, min_traces=2049),
+    dict(name="gl1_sarsa_m8192", algo="sarsa", M=8192, flow_seed=5, env=9, ticks=3000,
+         over={"learning.gamma": 1.0, "learning.lambda": 1.0}, trace_cap=8192, min_traces=513),
+    dict(name="m1_q", algo="q_learn", M=1, flow_seed=5, env=10, ticks=2000, over={}),
+]
+
+
+def learner_shape_runs():
+    import golden_util
+    cases = []
+    for c in LEARNER_SHAPE_CASES:
+        y = config.example_dict(**{"learning.memory_size": c["M"], "learning.algorithm": c["algo"], **c["over"]})
+        y_run = json.loads(json.dumps(y))
+        y_run["debug"]["random_seed"] = y["debug"]["random_seed"] + c["env"]
+        ref = ol.run_ref(y_run, c["flow_seed"], c["env"], c["ticks"])
+        recs = ref["records"]
+        with open(os.path.join(GOLD, "digests_%s.bin" % c["name"]), "wb") as f:
+            for r in recs:
+                f.write(golden_util.record_digest(r))
+        longest = max(r.n_traces for r in recs)
+        assert longest >= c.get("min_traces", 0) and longest <= c.get("max_traces", longest), (c["name"], longest)
+        cases.append(dict(c, yaml=y, trace_cap=c.get("trace_cap", 0), n_records=len(recs)))
+        print(c["name"], len(recs), "records; longest trace list", longest)
+    with open(os.path.join(GOLD, "learner_shapes.json"), "w") as f:
+        json.dump(cases, f, indent=1)
 
 
 def day_t0(cfg, open_ticks, dt_ms=250):
@@ -201,6 +246,7 @@ def main():
     with open(os.path.join(GOLD, "manifest.json"), "w") as f:
         json.dump(manifest, f, indent=1)
     tested_reference_runs()
+    learner_shape_runs()
 
 
 def tested_reference_runs():
@@ -246,4 +292,7 @@ def tested_reference_runs():
 
 
 if __name__ == "__main__":
-    main()
+    if sys.argv[1:] == ["learner_shapes"]:  # only digests_<learner shape>.bin and learner_shapes.json
+        learner_shape_runs()
+    else:
+        main()
